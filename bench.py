@@ -9,8 +9,9 @@ fused AdamW update of all 1.41 B parameters - replayed as one CUDA graph; data-p
   python bench.py --gpus N --steps K --warmup W                 -> one JSON line (rank 0)
   python bench.py --workload lora|zeroscope|vae ...             -> configs[2] / [3] / [4] of BASELINE.json (extra lines)
   python bench.py --impl reference ...                          -> the reference algorithm on the host CPU cores: the
-        reference's own models/*.py when /root/reference is present (build container), else the oracle port of it (GPU box);
-        its diffusers dependency cannot be installed here (DESIGN.md section 5), same metric/unit.
+        reference's own models/*.py when T2V_REFERENCE_ROOT names a checkout of it, else the oracle port of it;
+        its diffusers dependency is not installed (DESIGN.md section 5), same metric/unit.
+  python bench.py ... --dump-outputs DIR                        -> also writes the last timed step's outputs as DIR/*.npy
 Everything under oracle/ is used only for the parity / cpu_baseline / --impl reference legs.
 """
 import argparse
@@ -146,7 +147,7 @@ def oracle_pass(sd_cpu, cfg, inputs, threads):
 
 def reference_pass(Ref, sd_cpu, cfg, inputs, threads):
     """The same pass through the reference's UNMODIFIED models/unet_3d_condition.py + unet_3d_blocks.py (imported from
-    /root/reference over the diffusers stand-in, oracle/reference_import.py) with the step glue of train.py:751-834."""
+    T2V_REFERENCE_ROOT over the diffusers stand-in, oracle/reference_import.py) with the step glue of train.py:751-834."""
     from oracle import leaves as L
     torch.set_num_threads(threads)
     lat, noise, t, ehs = inputs
@@ -211,7 +212,7 @@ def run_reference(args):
     ms = 1e3 * sum(times) / len(times)
     fps = frames / (ms / 1e3)
     what = ("the reference's unmodified models/*.py over the diffusers stand-in" if Ref is not None else
-            "oracle port of the reference algorithm (/root/reference is absent on this box)")
+            "oracle port of the reference algorithm (T2V_REFERENCE_ROOT names no reference checkout)")
     line = {"impl": "reference", "metric": "finetune frames/sec (one UNet fwd+bwd pass per step)", "value": fps, "unit": "frames/s",
             "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup, "ms_per_step": ms, "higher_is_better": True,
             "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
@@ -263,6 +264,28 @@ def shutdown(world, step=None):
         dist.destroy_process_group()
     finally:
         os._exit(0)
+
+
+DUMP_SAMPLE = 1 << 22   # elements per sampled array: 16 MB in float32
+
+
+def dump_outputs(out_dir, loss, arena, optimizer):
+    """What the last step hands its caller: the loss, and the updated fp32 master weights and AdamW first moment (the
+    gradients without an optimizer), the latter two as the same fixed, seeded sample of the flat parameter arena."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    n = arena.master.numel()
+    idx = torch.randint(0, n, (min(n, DUMP_SAMPLE),), generator=torch.Generator().manual_seed(0)).sort().values
+    idx = idx.to(arena.master.device)
+    arrays = {"loss": np.array([loss], dtype=np.float64), "weights_sample": arena.master[idx]}
+    if optimizer is not None:
+        arrays["exp_avg_sample"] = optimizer.exp_avg[idx]
+    else:
+        arrays["grad_sample"] = arena.grad[idx]
+    for name, a in arrays.items():
+        if isinstance(a, torch.Tensor):
+            a = a.float().cpu().numpy()
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def time_events(fn, n):
@@ -347,14 +370,22 @@ def main():
     ap.add_argument("--profile-timed-region", action="store_true",
                     help="cudaProfilerStart/Stop around the K timed steps: `ncu --profile-from-start off ... python bench.py --steps 1 "
                          "--profile-timed-region` lists exactly the kernels of the timed region (numbers printed under ncu are not bench values)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed as DIR/<name>.npy (the loss and fixed seeded samples of the "
+                         "updated weights and of the optimizer's first moment), to compare two builds output for output")
     args = ap.parse_args()
+    if args.steps is not None and args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or args.workload == "vae"):
+        ap.error("--dump-outputs covers the finetune step (--impl ours, workloads cfg2 / lora / zeroscope)")
     world = int(os.environ.get("WORLD_SIZE", "1"))
-    if args.steps is None:
-        args.steps = 20 if world == 1 else 50   # collective-bound timings need more samples (round-1 verdict)
     if args.impl == "reference":
-        args.steps = min(args.steps, 3)
+        if args.steps is None:
+            args.steps = 3   # full-size fp32 passes on the host cores take tens of seconds each
         args.warmup = min(args.warmup, 1)
         return run_reference(args)
+    if args.steps is None:
+        args.steps = 20 if world == 1 else 50   # collective-bound timings need more samples
     args.warmup = max(args.warmup, 3)
 
     import torch.distributed as dist
@@ -488,6 +519,8 @@ def main():
     f1.record()
     barrier()
     ms_e2e = f0.elapsed_time(f1) / args.steps
+    if args.dump_outputs and rank == 0:   # before the optimizer is timed alone below: that moves the weights again
+        dump_outputs(args.dump_outputs, lv, step.arena, optimizer)
     # ---- the optimizer's share (clip + AdamW over the trainable set), timed alone on the device
     opt_ms = None
     if optimizer is not None:

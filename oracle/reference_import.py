@@ -1,15 +1,16 @@
-"""ORACLE helper: import the reference's own wiring files UNMODIFIED from /root/reference (read-only) on top of the
-diffusers stand-in.  Only usable where /root/reference exists (this container, not the GPU box)."""
+"""ORACLE helper: import the reference's own wiring files UNMODIFIED from a checkout of the reference (read-only) on top
+of the diffusers stand-in.  The checkout is named by T2V_REFERENCE_ROOT; the golden generators under tests/golden/ need
+it, the tests compare with the fixtures those generators stored."""
 import importlib
 import os
 import sys
 
-REFERENCE_ROOT = os.environ.get("T2V_REFERENCE_ROOT", "/root/reference")
+REFERENCE_ROOT = os.environ.get("T2V_REFERENCE_ROOT", "")
 _STANDIN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "diffusers_standin")
 
 
 def reference_available():
-    return os.path.isfile(os.path.join(REFERENCE_ROOT, "models", "unet_3d_condition.py"))
+    return bool(REFERENCE_ROOT) and os.path.isfile(os.path.join(REFERENCE_ROOT, "models", "unet_3d_condition.py"))
 
 
 def import_reference_unet():

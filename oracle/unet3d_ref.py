@@ -8,8 +8,8 @@ on top of the leaf restatements in oracle/leaves.py.  It consumes a plain state 
 parameter names (SURVEY.md appendix C), so it also checks the product's parameter naming.
 
 PARITY UNPINNED by the reference's own tests (there are none).  Pinned here by
-tests/test_oracle_vs_reference.py: the reference's models/*.py imported UNMODIFIED (over oracle/diffusers_standin)
-must reproduce this function's output on the same state dict, wherever /root/reference is present.
+tests/test_oracle_vs_reference.py: this function must reproduce the outputs that the reference's models/*.py, imported
+UNMODIFIED (over oracle/diffusers_standin), gave on the same state dict (tests/golden/oracle_vs_reference.pt).
 """
 import torch
 import torch.nn.functional as F

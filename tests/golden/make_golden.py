@@ -1,6 +1,6 @@
-"""Generates tests/golden/unet_small_*.pt from the REFERENCE's own wiring: /root/reference/models/*.py imported
-unmodified (over oracle/diffusers_standin, since diffusers is not installable here), fp32, CPU.
-Run in the build container only:  python tests/golden/make_golden.py
+"""Generates tests/golden/unet_small_*.pt from the REFERENCE's own wiring: its models/*.py imported
+unmodified (over oracle/diffusers_standin, since diffusers is not installed), fp32, CPU.  Needs a checkout of the reference:
+    T2V_REFERENCE_ROOT=<reference checkout> python tests/golden/make_golden.py
 The fixtures pin (a) the oracle restatement (tests/test_golden.py, CPU) and (b) the CUDA path (GPU) to the reference."""
 import os
 import sys

@@ -1,7 +1,7 @@
-"""Generates tests/golden/lora_*.pt from the REFERENCE's own LoRA code: /root/reference/utils/lora.py imported unmodified
-(LoraInjectedLinear / Conv2d / Conv3d, inject_trainable_lora_extended) and, for the model-level case, the reference's
-unmodified models/*.py over oracle/diffusers_standin.  fp32, CPU.  Run in the build container only:
-    python tests/golden/make_golden_lora.py
+"""Generates tests/golden/lora_module_*.pt and lora_unet_small_f4.pt from the REFERENCE's own LoRA code: its utils/lora.py
+imported unmodified (LoraInjectedLinear / Conv2d / Conv3d, inject_trainable_lora_extended) and, for the model-level case, the
+reference's unmodified models/*.py over oracle/diffusers_standin.  fp32, CPU.  Needs a checkout of the reference:
+    T2V_REFERENCE_ROOT=<reference checkout> python tests/golden/make_golden_lora.py
 The fixtures pin the B200 LoRA path (tests/test_lora_gpu.py) to the reference classes rather than to this repo's own wiring."""
 import contextlib
 import importlib.util
@@ -61,7 +61,7 @@ def module_cases(ref):
         dy = torch.randn(y.shape, generator=g)
         y.backward(dy)
         out[name] = dict(state={k: v.detach().clone() for k, v in m.state_dict().items()}, x=x.detach().clone(), y=y.detach().clone(), dy=dy,
-                         dx=x.grad.clone(), grads={n: p.grad.clone() for n, p in m.named_parameters() if p.grad is not None},
+                         dx=x.grad.clone(), grads={n: p.grad.clone() for n, p in m.named_parameters() if "lora" in n and p.grad is not None},
                          scale=m.scale, r=m.lora_down.weight.shape[0])
     return out
 
@@ -96,9 +96,10 @@ def model_case(ref):
 def main():
     torch.set_num_threads(8)
     ref = ref_lora()
-    path = os.path.join(ROOT, "tests", "golden", "lora_modules.pt")
-    torch.save(module_cases(ref), path)
-    print("lora_modules", os.path.getsize(path) // 1024, "KiB")
+    for name, case in module_cases(ref).items():   # one file per case keeps each fixture small
+        path = os.path.join(ROOT, "tests", "golden", f"lora_module_{name}.pt")
+        torch.save(case, path)
+        print("lora_module_" + name, os.path.getsize(path) // 1024, "KiB")
     path = os.path.join(ROOT, "tests", "golden", "lora_unet_small_f4.pt")
     torch.save(model_case(ref), path)
     print("lora_unet_small_f4", os.path.getsize(path) // 1024, "KiB")

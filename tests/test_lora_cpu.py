@@ -1,8 +1,8 @@
 """cloneofsimo LoRA surface (utils/lora.py, utils/lora_handler.py) on CPU with emulated primitives:
-injection census and key names against the reference's own injector (where /root/reference exists), module-level
-forward parity against the reference classes, zero-init identity, and the collapse/remove round trip."""
+injection census and key names against the reference's own injector, module-level forward parity against the reference
+classes (both from tests/golden/lora_reference.pt, made by tests/golden/make_golden_reference.py with the reference's
+utils/lora.py imported unmodified), zero-init identity, and the collapse/remove round trip."""
 import contextlib
-import importlib.util
 import io
 import os
 
@@ -11,9 +11,9 @@ import torch
 
 from helpers import emulated_prims, rel_l2, seeded_state_dict
 from oracle import ops_ref
-from oracle.reference_import import REFERENCE_ROOT, import_reference_unet, reference_available
 
 SMALL = dict(block_out_channels=(64, 128, 128, 128), attention_head_dim=64, cross_attention_dim=64)
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "lora_reference.pt")
 
 
 @pytest.fixture(autouse=True)
@@ -36,56 +36,44 @@ def _model(seed=0):
     return m.eval(), sd
 
 
-def _ref_lora():
-    spec = importlib.util.spec_from_file_location("_t2v_ref_lora", os.path.join(REFERENCE_ROOT, "utils", "lora.py"))
-    mod = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(mod)
-    return mod
+def _golden():
+    return torch.load(GOLDEN, weights_only=False)
 
 
-@pytest.mark.skipif(not reference_available(), reason="reference sources not present")
 def test_injection_matches_reference_injector():
     from t2v_b200.utils import lora as mylora
-    ref = _ref_lora()
+    ref = _golden()["injection"]
+    assert ref["cfg"] == SMALL
     m, sd = _model()
-    r = import_reference_unet()(**SMALL)
-    r.load_state_dict(sd)
     with _quiet():
-        pm, nm = mylora.inject_trainable_lora_extended(m, {"UNet3DConditionModel"}, r=16)
-        pr, nr = ref.inject_trainable_lora_extended(r, {"UNet3DConditionModel"}, r=16)
-    assert len(pm) == len(pr) and sorted(nm) == sorted(nr)
+        pm, nm = mylora.inject_trainable_lora_extended(m, {"UNet3DConditionModel"}, r=ref["r"])
+    assert len(pm) == ref["n_param_groups"] and sorted(nm) == ref["names"]
     a = {k: tuple(v.shape) for k, v in m.named_parameters()}
-    b = {k: tuple(v.shape) for k, v in r.named_parameters()}
-    assert a == b
-    kinds = lambda mod, lib: sorted(type(x).__name__ for x in mod.modules() if type(x).__name__.startswith("LoraInjected"))
-    assert kinds(m, mylora) == kinds(r, ref)
+    assert a == ref["shapes"]
+    kinds = sorted(type(x).__name__ for x in m.modules() if type(x).__name__.startswith("LoraInjected"))
+    assert kinds == ref["kinds"]
     # zero-initialised up, N(0, 1/r) down, shared base parameters, default dropout (0.1 / 0.1 / 0)
     w = m.down_blocks[0].resnets[0].conv1
     assert isinstance(w, mylora.LoraInjectedConv2d) and w.lora_up.weight.abs().max() == 0 and w.dropout.p == 0.1
     assert m.down_blocks[0].temp_convs[0].conv1[2].dropout.p == 0
 
 
-@pytest.mark.skipif(not reference_available(), reason="reference sources not present")
 def test_wrapper_forward_matches_reference_classes():
     from t2v_b200.utils import lora as mylora
-    ref = _ref_lora()
-    torch.manual_seed(0)
+    ref = _golden()["wrappers"]
     with _quiet():
-        lr_, lm = ref.LoraInjectedLinear(64, 128, True, r=16), mylora.LoraInjectedLinear(64, 128, True, r=16)
-        cr, cm = ref.LoraInjectedConv2d(64, 96, 3, 1, 1, r=16), mylora.LoraInjectedConv2d(64, 96, 3, 1, 1, r=16)
-        tr, tm = ref.LoraInjectedConv3d(64, 64, (3, 1, 1), (1, 0, 0), bias=True, r=16), mylora.LoraInjectedConv3d(64, 64, (3, 1, 1), (1, 0, 0), bias=True, r=16)
-    for a, b in ((lr_, lm), (cr, cm), (tr, tm)):
-        a.lora_up.weight.data.normal_(0, 0.1)
-        b.load_state_dict(a.state_dict())
-        a.eval(), b.eval()
-    x = torch.randn(50, 64)
-    xi = torch.randn(2, 64, 8, 8)
-    xv = torch.randn(1, 64, 5, 4, 4)
+        mods = dict(linear=mylora.LoraInjectedLinear(64, 128, True, r=16), conv2d=mylora.LoraInjectedConv2d(64, 96, 3, 1, 1, r=16),
+                    conv3d=mylora.LoraInjectedConv3d(64, 64, (3, 1, 1), (1, 0, 0), bias=True, r=16))
+    for name, m in mods.items():
+        m.load_state_dict(seeded_state_dict(m, ref[name]["weight_seed"]))
+        m.eval()
+    lm, cm, tm = mods["linear"], mods["conv2d"], mods["conv3d"]
+    x, xi, xv = ref["linear"]["x"], ref["conv2d"]["x"], ref["conv3d"]["x"]
     with emulated_prims():
-        assert rel_l2(lm(x), lr_(x)) < 1e-6
-        assert rel_l2(cm(xi.permute(0, 2, 3, 1).contiguous()).permute(0, 3, 1, 2), cr(xi)) < 1e-5
+        assert rel_l2(lm(x), ref["linear"]["y"]) < 1e-6
+        assert rel_l2(cm(xi.permute(0, 2, 3, 1).contiguous()).permute(0, 3, 1, 2), ref["conv2d"]["y"]) < 1e-5
         y = tm(xv.permute(0, 2, 3, 4, 1).reshape(1, 5, 16, 64).contiguous())
-        assert rel_l2(y.reshape(1, 5, 4, 4, 64).permute(0, 4, 1, 2, 3), tr(xv)) < 1e-5
+        assert rel_l2(y.reshape(1, 5, 4, 4, 64).permute(0, 4, 1, 2, 3), ref["conv3d"]["y"]) < 1e-5
 
 
 def test_zero_init_identity_and_collapse_round_trip():

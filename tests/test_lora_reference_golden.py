@@ -1,7 +1,7 @@
 """LoRA path against the REFERENCE's own classes (SURVEY 8 row a12).
 
-tests/golden/lora_*.pt were produced by /root/reference/utils/lora.py (LoraInjectedLinear / Conv2d / Conv3d and
-inject_trainable_lora_extended, imported unmodified - tests/golden/make_golden_lora.py) on the reference's models/*.py, so
+tests/golden/lora_module_*.pt and lora_unet_small_f4.pt were produced by the reference's utils/lora.py (LoraInjectedLinear /
+Conv2d / Conv3d and inject_trainable_lora_extended, imported unmodified - tests/golden/make_golden_lora.py) on the reference's models/*.py, so
 these cases pin the LoRA path to the reference implementation, not to this repo's own wiring (round-1 verdict).
 CPU variants run the host wiring over the emulated primitives (fp32); GPU variants run the CUDA kernels (bf16 tolerances)."""
 import contextlib
@@ -44,7 +44,7 @@ def test_lora_wrappers_match_reference_classes(name, device):
     """y and the gradients w.r.t. x, lora_up, lora_down of one wrapped layer vs the reference wrapper's own autograd."""
     from t2v_b200 import ops
     from t2v_b200.utils import lora as mylora
-    c = torch.load(os.path.join(GOLDEN, "lora_modules.pt"), weights_only=False)[name]
+    c = torch.load(os.path.join(GOLDEN, f"lora_module_{name}.pt"), weights_only=False)
     st = c["state"]
     r, scale = c["r"], c["scale"]
     if name.startswith("linear"):

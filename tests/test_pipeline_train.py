@@ -102,27 +102,23 @@ def test_raw_video_training_gpu(tmp_path):
 
 
 def test_reference_yaml_configs_load_into_main():
-    """Every shipped v2 YAML of the reference maps onto train.main's keyword surface (no unknown keys, no missing required)."""
-    import yaml
+    """Every shipped v2 YAML of the reference maps onto train.main's keyword surface (no unknown keys, no missing required).
+    tests/golden/reference_configs.json holds each YAML's top-level keys, dataset_types and train_data section
+    (tests/golden/make_golden_reference.py)."""
     from t2v_b200 import train
-    cfg_dir = "/root/reference/configs/v2"
-    if not os.path.isdir(cfg_dir):
-        pytest.skip("reference configs not present")
+    with open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_configs.json")) as f:
+        configs = json.load(f)
     sig = inspect.signature(train.main)
     names = set(sig.parameters)
     seen = 0
-    for fn in sorted(os.listdir(cfg_dir)):
-        if not fn.endswith(".yaml"):
-            continue
-        with open(os.path.join(cfg_dir, fn)) as f:
-            cfg = yaml.safe_load(f)
-        unknown = sorted(set(cfg) - names)
+    for fn, cfg in sorted(configs.items()):
+        unknown = sorted(set(cfg["keys"]) - names)
         assert not unknown, (fn, unknown)
-        sig.bind_partial(**cfg)
+        sig.bind_partial(**dict.fromkeys(cfg["keys"]))
         # the `train_data:` section constructs every dataset class it names
         from t2v_b200.utils import dataset as D
-        for kind in cfg.get("dataset_types", []):
+        for kind in cfg["dataset_types"]:
             assert kind in D.DATASETS, (fn, kind)
-            D.DATASETS[kind](**dict(cfg.get("train_data") or {}), tokenizer=None)
+            D.DATASETS[kind](**dict(cfg["train_data"]), tokenizer=None)
         seen += 1
     assert seen >= 1
